@@ -49,7 +49,14 @@ def parse():
     ap.add_argument("--no-reference-gpu", action="store_true", help="skip the reference-GPU leg (the unmodified reference step timed on this GPU after our arm, N=1 only)")
     ap.add_argument("--no-cuda-graphs", action="store_true", help="enqueue every step eagerly instead of replaying one captured CUDA graph of the whole step "
                          "(the reference driver's --cuda_graphs, run_pretraining.py:602-640,669)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed resident pass, write what its last step computed as DIR/<name>.npy "
+                         "(float32, see dump_outputs); inputs and weights are seeded, so two builds run with the same arguments can be compared array by array")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
 
 
 def peaks():
@@ -96,6 +103,42 @@ class ClockSampler:
         reasons = [n for i, n in enumerate(names) if any(r[4 + i].lower().startswith("active") for r in rows)]
         return {"sm_mhz": sm[len(sm) // 2], "sm_max_mhz": float(rows[0][2]), "power_w_max": max(float(r[3]) for r in rows),
                 "samples": len(rows), "reasons": reasons}
+
+
+def dump_outputs(out_dir, model, opt, loss, per_tensor=4096):
+    """Write what one training step hands its caller, as float32 .npy files in out_dir:
+      loss.npy               the step's loss, shape [1]
+      global_grad_norm.npy   the optimizer's global gradient norm of that step, shape [1]
+      params.npy, master_params.npy, exp_avg.npy, exp_avg_sq.npy
+                             every parameter the step updated (named_parameters() order) after the update: the 16-bit model weights,
+                             their fp32 masters and the two moments, each sampled at the same at most `per_tensor` positions and concatenated.
+    The positions come from a fixed seed and the tensor sizes only, so they are the same in every run; for BERT-large
+    (398 tensors) each array holds about 0.94M values, about 14 MB in all.  Compare two builds with a tolerance: split-K GEMMs
+    accumulate with fp32 atomics in no fixed order, so two runs of one build already differ slightly (on a B200 at its 1000 W
+    limit, the loss of the default workload by 4e-5 relative)."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    net = model.module if hasattr(model, "module") else model
+    masters = {id(p): m for g, g32 in zip(opt.param_groups, opt.param_groups_fp32) for p, m in zip(g["params"], g32["params"])}
+    gen = torch.Generator().manual_seed(0)
+    cols = {"params": [], "master_params": [], "exp_avg": [], "exp_avg_sq": []}
+    for _, p in net.named_parameters():
+        st = opt.state.get(p, {})
+        if "exp_avg" not in st:                     # no gradient, so the step did not touch it
+            continue
+        n = p.numel()
+        idx = (torch.randperm(n, generator=gen)[:per_tensor].sort().values if n > per_tensor else torch.arange(n)).to(p.device)
+        master = masters.get(id(p))
+        for name, t in (("params", p), ("master_params", p if master is None else master),
+                        ("exp_avg", st["exp_avg"]), ("exp_avg_sq", st["exp_avg_sq"])):
+            cols[name].append(t.detach().reshape(-1)[idx].float().cpu())
+    arrays = {k: torch.cat(v).numpy() for k, v in cols.items()}
+    arrays["loss"] = loss.detach().float().reshape(1).cpu().numpy()
+    arrays["global_grad_norm"] = opt._global_grad_norm.detach().float().reshape(1).cpu().numpy()
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+    log(f"wrote {len(arrays)} arrays ({sum(a.nbytes for a in arrays.values()) / 2**20:.1f} MB) to {out_dir}")
 
 
 # ------------------------------------------------------------------------------------------------
@@ -231,7 +274,7 @@ def run_reference(args):
         return
     cfg, S, B, P = workload(args)
     ref_batch = args.ref_batch or 2
-    steps, warm = max(1, min(args.steps, 4)), max(0, min(args.warmup, 1))
+    steps, warm = args.steps, args.warmup
     r = cpu_reference_run(cfg, S, P, ref_batch, steps, warm)
     n = args.gpus
     line = {"impl": "reference", "metric": METRIC, "value": round(r["value"], 4), "unit": "sequences/s", "n_gpus": n, "steps": steps,
@@ -384,6 +427,8 @@ def run_ours(args):
     torch.cuda.profiler.stop()
     torch.cuda.nvtx.range_pop()
     log(f"resident pass: {ms_res / args.steps:.2f} ms/step")
+    if args.dump_outputs and rank == 0:            # before the passes below train the model further
+        dump_outputs(args.dump_outputs, model, opt, graph["loss"])
     launches = (L.launch_count["n"] - n0) if launches_per_step is None else launches_per_step * args.steps
     ms_e2e, host_e2e = timed(step_e2e, args.steps)
     log(f"e2e pass: {ms_e2e / args.steps:.2f} ms/step")

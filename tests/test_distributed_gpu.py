@@ -74,7 +74,7 @@ def _worker(rank, world, port, dtype_name, out_path):
 @pytest.mark.parametrize("dtype_name,tol", [("float32", 1e-5), ("bfloat16", 2e-2)])
 def test_two_rank_ddp_step_equals_one_rank_step_on_concatenated_batch(tmp_path, dtype_name, tol):
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs (gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     import torch.multiprocessing as mp
     from deeplearningexamples_b200 import training as T
     out = str(tmp_path / "rank0.pt")

@@ -26,7 +26,7 @@ SMALL = dict(attention_probs_dropout_prob=0.1, hidden_act="gelu", hidden_dropout
 
 def _need_ref():
     if not os.path.exists(os.path.join(REF, "run_pretraining.py")):
-        pytest.skip("baseline/_ref/BERT not installed (python baseline/install_ref.py where /root/reference exists)")
+        pytest.skip("baseline/_ref/BERT not installed (python baseline/install_ref.py where the reference tree exists)")
 
 
 def _run(arm, out, extra, steps, tmp_path, timeout=600):
