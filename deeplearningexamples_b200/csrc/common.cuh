@@ -306,6 +306,29 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
     }
 }
 __device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+// arrive on an mbarrier given by its shared::cluster address (mapa_shared), e.g. one in the peer CTA of a pair
+__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
+    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
+}
+
+// ---------------------------------------------------------------------------------------------
+// clusters
+// ---------------------------------------------------------------------------------------------
+__device__ __forceinline__ uint32_t cluster_ctarank() {
+    uint32_t r;
+    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
+    return r;
+}
+// every thread of every CTA of the cluster: arrive (release) + wait (acquire)
+__device__ __forceinline__ void cluster_sync() {
+    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// shared::cluster address of the variable at the same offset in CTA `rank` of the cluster
+__device__ __forceinline__ uint32_t mapa_shared(uint32_t smem_addr, uint32_t rank) {
+    uint32_t r;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(rank));
+    return r;
+}
 // generic-proxy smem writes -> visible to the async proxy (TMA / tcgen05 operand reads)
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
@@ -319,6 +342,14 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
     asm volatile(
         "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
         ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
+        : "memory");
+}
+// CTA-pair form (tcgen05 cta_group::2): the data lands in THIS CTA's shared memory, the completed bytes are counted on the mbarrier at
+// `bar_cluster` (a shared::cluster address, which may lie in the peer CTA)
+__device__ __forceinline__ void tma_load_2d_pair(void* smem_dst, const CUtensorMap* m, uint32_t bar_cluster, int c0, int c1) {
+    asm volatile(
+        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+        ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster), "r"(c0), "r"(c1)
         : "memory");
 }
 __device__ __forceinline__ void tma_load_3d(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2) {
@@ -364,6 +395,32 @@ __device__ __forceinline__ void umma_bf16_ss(uint32_t tmem_d, uint64_t desc_a, u
         ".reg .pred p;\n"
         "setp.ne.b32 p, %4, 0;\n"
         "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n"
+        "}\n" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
+}
+// CTA-pair (cta_group::2) forms.  All tcgen05 instructions of one kernel must use the same cta_group.  alloc / relinquish / dealloc
+// are executed collectively by one warp of EACH CTA of the pair and give both CTAs the same TMEM address.  The MMA is issued by the
+// even CTA only: A (M = 256) is its 128 rows in each CTA's shared memory, B is N/2 rows in each, at the same offsets, and each CTA's
+// TMEM receives its own 128 rows of D.
+__device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_result, uint32_t ncols) {
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_result)), "r"(ncols) : "memory");
+}
+__device__ __forceinline__ void tmem_relinquish_pair() {
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+// arrive on the mbarrier at this offset in BOTH CTAs of the pair once all previously issued MMAs have completed
+__device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
+    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+                 ::"r"(smem_u32(bar)), "h"((uint16_t)0x3) : "memory");
+}
+__device__ __forceinline__ void umma_bf16_ss_pair(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n"
+        ".reg .pred p;\n"
+        "setp.ne.b32 p, %4, 0;\n"
+        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n"
         "}\n" ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
 }
 // D[tmem] (+)= A[tmem] * B[smem]

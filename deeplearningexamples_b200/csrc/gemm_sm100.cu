@@ -1,9 +1,15 @@
-// Dense bf16 GEMM for sm_100a: tcgen05.mma (cta_group::1, M=128) with fp32 accumulators in TMEM,
-// operands staged by TMA into 128B-swizzled shared memory, persistent warp-specialised CTAs
-// (1 TMA producer warp, 1 MMA issuer warp, 8 epilogue warps), double-buffered accumulators so the
+// Dense bf16 GEMM for sm_100a: tcgen05.mma on CTA pairs (cta_group::2, M = 256) with fp32 accumulators in TMEM,
+// operands staged by TMA into 128B-swizzled shared memory, persistent warp-specialised CTAs launched in clusters of 2
+// (1 TMA producer warp, 1 MMA issuer warp, 8 or 16 epilogue warps per CTA), double-buffered accumulators so the
 // epilogue of tile i overlaps the main loop of tile i+1.
 //
 //   D[M,N] = A[M,K] * B[N,K]^T     (K = reduction)
+//
+// A work unit is a 256 x BN output tile (and a K range, under split-K) shared by the two CTAs of a cluster: the even CTA
+// owns rows 0-127 of the tile, the odd CTA rows 128-255.  Each CTA loads its own 128 rows of A and HALF of B (BN/2 rows),
+// so per flop an SM moves a third less operand data out of L2 and reads a third less shared memory for the MMA than a
+// 128 x BN tile per SM; one 256 x BN x 16 MMA issued by the even CTA serves both SMs, and each SM's TMEM receives its
+// own 128 rows of D.
 //
 // Either operand may be "K-major" (row-major [rows, K], the reduction dim contiguous) or
 // "MN-major" (row-major [K, rows], the M/N dim contiguous) so forward (x W^T), dgrad (dy W) and
@@ -25,14 +31,14 @@
 
 namespace dle {
 
-constexpr int BM = 128;
+constexpr int BM = 128;      // rows of a tile per CTA; a pair tile has 2 * BM
 constexpr int BK = 64;        // 64 bf16 = 128 B = one swizzle row
 constexpr int UMMA_K = 16;
 // Epilogue warps (template parameter EW): 8 (two per TMEM lane quarter, each draining half the columns) or 16 (four per quarter, a
-// quarter of the columns each, 3 pipeline stages instead of 4 to pay for their staging tiles, <= 104 registers per thread).
-// Measured at T = 65536 (profiles/r02_gemm_microbench_run7_*.log): 16 warps lift the gelu'(u)-times-dgrad epilogue (817 instructions per
-// 32x32 chunk, the accumulator waiting on the epilogue) from 950 to 1055 TFLOP/s, and cost every other shape 3-15 % -- the third stage
-// alone costs the K = 4096 shapes 8 % -- so only DLE_EPI_DGELU launches take the 16-warp instance.
+// quarter of the columns each, <= 104 registers per thread).  With one 128 x BN tile per SM (a 48 KB stage at BN = 256) the 16-warp
+// instance had to drop to 3 stages and only paid for the gelu'(u)-times-dgrad epilogue (profiles/r02_gemm_microbench_run7_*.log); a
+// CTA's share of a pair stage is 32 KB, so 16 warps now cost one stage of six, not one of four.  Which epilogues take 16 warps:
+// DLE_GEMM_EW16_EPILOGUES (bit mask over DLE_EPI_*; a compile-time switch so that variants can be built and measured side by side).
 // Warp roles: epilogue warps 0..EW-1, then TMA, MMA, TMEM alloc (+ a spare with 8).  The single-issuer warps carry the HIGHEST
 // warp ids: the SM sub-partition arbiter favours higher warp ids, and a starved MMA issuer idles the tensor pipe.
 template <int BN, int EW> struct GemmCfg {
@@ -41,20 +47,25 @@ template <int BN, int EW> struct GemmCfg {
     static constexpr int EPI_PARTS = EW / 4;                        // column parts per tile (one per warp of a quarter)
     static constexpr int THREADS = (EW == 8) ? 384 : 608;
     static constexpr int WARP_TMA = EW, WARP_MMA = EW + 1, WARP_ALLOC = EW + 2;
-    static constexpr int A_BYTES = BM * BK * 2;
-    static constexpr int B_BYTES = BN * BK * 2;
-    static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-    static constexpr int STAGES = (BN == 256) ? (EW == 8 ? 4 : 3) : (EW == 8 ? 6 : 4);
-    static constexpr int TMEM_COLS = 2 * BN;            // double-buffered accumulator
+    static constexpr int A_BYTES = BM * BK * 2;                     // this CTA's 128 rows of A
+    static constexpr int B_BYTES = (BN / 2) * BK * 2;               // this CTA's half of B
+    static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;           // per CTA; a pair stage is twice this
+    static constexpr int STAGES = (BN == 256) ? (EW == 8 ? 6 : 5) : (EW == 8 ? 8 : 6);
+    static constexpr int TMEM_COLS = 2 * BN;            // double-buffered accumulator (128 lanes x BN columns each, in each CTA)
     // epilogue: per warp a 2 KB output staging tile + a 2 KB cp.async landing tile for the residual / pre-activation operand,
     // plus 3 x 2 x 256 B of bias staging (triple-buffered per tile, one slice per column half)
     static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + EPI_WARPS * 2048 + EPI_WARPS * 2048 + 1536 + 1024 /*align slack*/ + 256 /*barriers*/;
     static_assert(SMEM_BYTES <= 232448, "shared memory budget");
+    static_assert((2 * STAGES + 4) * 8 + 4 <= 256, "barrier area");
 };
+
+#ifndef DLE_GEMM_EW16_EPILOGUES
+#define DLE_GEMM_EW16_EPILOGUES (1u << DLE_EPI_DGELU)
+#endif
 
 struct GemmKernelParams {
     int M, N, K;
-    int m_tiles, n_tiles, splits, kb_total;
+    int m_tiles, n_tiles, splits, kb_total;   // m_tiles: 256-row pair tiles
     int epilogue;
     const bf16* bias;      // [N] or null
     const bf16* aux;       // [M, ld_aux] residual / pre-activation, or null
@@ -276,25 +287,28 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
     uint8_t* epi_stage = smem + Cfg::STAGES * Cfg::STAGE_BYTES;                 // 8 warps x (out tile, aux tile), then the bias slices
     uint8_t* epi_bias = epi_stage + 2 * EPI_WARPS * EPI_TILE_BYTES;
     uint64_t* bars = reinterpret_cast<uint64_t*>(epi_bias + EPI_BIAS_BYTES);
-    uint64_t* full_bar = bars;                         // [STAGES]  TMA -> MMA
-    uint64_t* empty_bar = bars + Cfg::STAGES;          // [STAGES]  MMA -> TMA
-    uint64_t* tmem_full = bars + 2 * Cfg::STAGES;      // [2]       MMA -> epilogue
-    uint64_t* tmem_empty = bars + 2 * Cfg::STAGES + 2; // [2]       epilogue -> MMA
+    // Barriers exist in both CTAs at the same offsets; full_bar and tmem_empty are only used in the even (leader) CTA.
+    uint64_t* full_bar = bars;                         // [STAGES]  TMA of both CTAs -> MMA
+    uint64_t* empty_bar = bars + Cfg::STAGES;          // [STAGES]  MMA -> TMA of each CTA (multicast commit)
+    uint64_t* tmem_full = bars + 2 * Cfg::STAGES;      // [2]       MMA -> epilogue of each CTA (multicast commit)
+    uint64_t* tmem_empty = bars + 2 * Cfg::STAGES + 2; // [2]       epilogue warps of both CTAs -> MMA
     uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(bars + 2 * Cfg::STAGES + 4);
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
+    const uint32_t rank = cluster_ctarank();           // 0: rows 0-127 of every pair tile, issues the MMAs; 1: rows 128-255
+    const int pair = blockIdx.x >> 1, num_pairs = gridDim.x >> 1;
 
     if (threadIdx.x == 0) {
         tma_prefetch_desc(&tmap_a);
         tma_prefetch_desc(&tmap_b);
         for (int s = 0; s < Cfg::STAGES; ++s) { mbar_init(&full_bar[s], 1); mbar_init(&empty_bar[s], 1); }
-        for (int s = 0; s < 2; ++s) { mbar_init(&tmem_full[s], 1); mbar_init(&tmem_empty[s], EPI_WARPS); }
+        for (int s = 0; s < 2; ++s) { mbar_init(&tmem_full[s], 1); mbar_init(&tmem_empty[s], 2 * EPI_WARPS); }
         fence_barrier_init();
     }
-    if (warp == WARP_ALLOC) { tmem_alloc(tmem_ptr, Cfg::TMEM_COLS); tmem_relinquish(); }
+    if (warp == WARP_ALLOC) { tmem_alloc_pair(tmem_ptr, Cfg::TMEM_COLS); tmem_relinquish_pair(); }
     tc_fence_before();
-    __syncthreads();
+    cluster_sync();                                    // the peer's barriers are initialised before anything signals them
     tc_fence_after();
     const uint32_t tmem_base = *tmem_ptr;
 
@@ -306,79 +320,89 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
     // registers and wraps every UTCHMMA / UTMALDG in an ELECT + R2UR + BRA.U.ANY waterfall (11-16 instructions per MMA, measured on the
     // attention kernels as an MMA-issue-bound tensor pipe at 18 %); warp-uniform flow issues consecutive MMAs back to back.
     if (warp == WARP_TMA) {
-        // ===================== TMA producer =====================
+        // ===================== TMA producer (both CTAs; completions counted on the leader's full_bar) =====================
         int stage = 0; uint32_t phase = 0;
-        for (int unit = blockIdx.x; unit < total_units; unit += gridDim.x) {
+        for (int unit = pair; unit < total_units; unit += num_pairs) {
             const int tile = unit / p.splits, split = unit - tile * p.splits;
-            const int m_blk = tile / p.n_tiles, n_blk = tile - m_blk * p.n_tiles;
+            const int m_pair = tile / p.n_tiles, n_blk = tile - m_pair * p.n_tiles;
+            const int row0 = (m_pair * 2 + (int)rank) * BM, col0 = n_blk * BN + (int)rank * (BN / 2);
             const int kb0 = split * kb_per_split, kb1 = min(p.kb_total, kb0 + kb_per_split);
             for (int kb = kb0; kb < kb1; ++kb) {
                 mbar_wait(&empty_bar[stage], phase ^ 1);
                 if (elect_one()) {
-                    mbar_expect_tx(&full_bar[stage], Cfg::STAGE_BYTES);
+                    const uint32_t fb = mapa_shared(smem_u32(&full_bar[stage]), 0);
+                    if (rank == 0) mbar_expect_tx(&full_bar[stage], 2 * Cfg::STAGE_BYTES);   // both CTAs' bytes
                     uint8_t* sa = smem + stage * Cfg::STAGE_BYTES;
                     uint8_t* sb = sa + Cfg::A_BYTES;
                     if (!A_MN) {
-                        tma_load_2d(sa, &tmap_a, &full_bar[stage], kb * BK, m_blk * BM);
+                        tma_load_2d_pair(sa, &tmap_a, fb, kb * BK, row0);
                     } else {
 #pragma unroll
                         for (int g = 0; g < BM / 64; ++g)
-                            tma_load_2d(sa + g * (BK * 128), &tmap_a, &full_bar[stage], m_blk * BM + g * 64, kb * BK);
+                            tma_load_2d_pair(sa + g * (BK * 128), &tmap_a, fb, row0 + g * 64, kb * BK);
                     }
                     if (!B_MN) {
-                        tma_load_2d(sb, &tmap_b, &full_bar[stage], kb * BK, n_blk * BN);
+                        tma_load_2d_pair(sb, &tmap_b, fb, kb * BK, col0);
                     } else {
 #pragma unroll
-                        for (int g = 0; g < BN / 64; ++g)
-                            tma_load_2d(sb + g * (BK * 128), &tmap_b, &full_bar[stage], n_blk * BN + g * 64, kb * BK);
+                        for (int g = 0; g < BN / 128; ++g)
+                            tma_load_2d_pair(sb + g * (BK * 128), &tmap_b, fb, col0 + g * 64, kb * BK);
                     }
                 }
                 __syncwarp();
                 if (++stage == Cfg::STAGES) { stage = 0; phase ^= 1; }
             }
         }
+        // The leader's MMA commits still arrive on this CTA's empty_bar after the last load: wait for every stage in flight so that
+        // no commit targets the shared memory of a CTA that has exited.
+        for (int s = 0; s < Cfg::STAGES; ++s) {
+            mbar_wait(&empty_bar[stage], phase ^ 1);
+            if (++stage == Cfg::STAGES) { stage = 0; phase ^= 1; }
+        }
     } else if (warp == WARP_MMA) {
-        // ===================== MMA issuer (one elected lane issues; the warp waits together) =====================
-        constexpr uint32_t idesc = make_idesc_bf16(BM, BN, A_MN, B_MN);
-        int stage = 0; uint32_t phase = 0; int it = 0;
-        const uint32_t smem_base = smem_u32(smem);
-        for (int unit = blockIdx.x; unit < total_units; unit += gridDim.x, ++it) {
-            const int split = unit % p.splits;
-            const int kb0 = split * kb_per_split, kb1 = min(p.kb_total, kb0 + kb_per_split);
-            const int acc = it & 1; const uint32_t acc_phase = (it >> 1) & 1;
-            mbar_wait(&tmem_empty[acc], acc_phase ^ 1);
-            tc_fence_after();
-            const uint32_t tmem_d = tmem_base + acc * BN;
-            for (int kb = kb0; kb < kb1; ++kb) {
-                mbar_wait(&full_bar[stage], phase);
+        // ===================== MMA issuer (leader CTA only; one elected lane issues, the warp waits together) =====================
+        if (rank == 0) {
+            constexpr uint32_t idesc = make_idesc_bf16(2 * BM, BN, A_MN, B_MN);
+            int stage = 0; uint32_t phase = 0; int it = 0;
+            const uint32_t smem_base = smem_u32(smem);
+            for (int unit = pair; unit < total_units; unit += num_pairs, ++it) {
+                const int split = unit % p.splits;
+                const int kb0 = split * kb_per_split, kb1 = min(p.kb_total, kb0 + kb_per_split);
+                const int acc = it & 1; const uint32_t acc_phase = (it >> 1) & 1;
+                mbar_wait(&tmem_empty[acc], acc_phase ^ 1);
                 tc_fence_after();
-                if (elect_one()) {
-                    const uint32_t sa = smem_base + stage * Cfg::STAGE_BYTES;
-                    const uint32_t sb = sa + Cfg::A_BYTES;
+                const uint32_t tmem_d = tmem_base + acc * BN;
+                for (int kb = kb0; kb < kb1; ++kb) {
+                    mbar_wait(&full_bar[stage], phase);
+                    tc_fence_after();
+                    if (elect_one()) {
+                        const uint32_t sa = smem_base + stage * Cfg::STAGE_BYTES;
+                        const uint32_t sb = sa + Cfg::A_BYTES;
 #pragma unroll
-                    for (int k = 0; k < BK / UMMA_K; ++k) {
-                        // K-major:  rows of 128 B, 8-row groups 1024 B apart (SBO); advance 32 B per UMMA_K.
-                        // MN-major: k-rows of 128 B (64 m/n elements), 8-k-row groups 1024 B apart (SBO),
-                        //           next 64 m/n elements BK*128 B further (LBO); advance 16 k-rows = 2048 B.
-                        const uint64_t da = A_MN ? make_smem_desc_sw128(sa + k * (UMMA_K * 128), BK * 128, 1024)
-                                                 : make_smem_desc_sw128(sa + k * (UMMA_K * 2), 0, 1024);
-                        const uint64_t db = B_MN ? make_smem_desc_sw128(sb + k * (UMMA_K * 128), BK * 128, 1024)
-                                                 : make_smem_desc_sw128(sb + k * (UMMA_K * 2), 0, 1024);
-                        umma_bf16_ss(tmem_d, da, db, idesc, (kb > kb0 || k > 0) ? 1u : 0u);
+                        for (int k = 0; k < BK / UMMA_K; ++k) {
+                            // K-major:  rows of 128 B, 8-row groups 1024 B apart (SBO); advance 32 B per UMMA_K.
+                            // MN-major: k-rows of 128 B (64 m/n elements), 8-k-row groups 1024 B apart (SBO),
+                            //           next 64 m/n elements BK*128 B further (LBO); advance 16 k-rows = 2048 B.
+                            const uint64_t da = A_MN ? make_smem_desc_sw128(sa + k * (UMMA_K * 128), BK * 128, 1024)
+                                                     : make_smem_desc_sw128(sa + k * (UMMA_K * 2), 0, 1024);
+                            const uint64_t db = B_MN ? make_smem_desc_sw128(sb + k * (UMMA_K * 128), BK * 128, 1024)
+                                                     : make_smem_desc_sw128(sb + k * (UMMA_K * 2), 0, 1024);
+                            umma_bf16_ss_pair(tmem_d, da, db, idesc, (kb > kb0 || k > 0) ? 1u : 0u);
+                        }
+                        umma_commit_pair(&empty_bar[stage]);      // frees this smem stage in both CTAs when the MMAs retire
+                        if (kb + 1 == kb1) umma_commit_pair(&tmem_full[acc]);     // accumulator complete -> both epilogues
                     }
-                    umma_commit(&empty_bar[stage]);      // frees this smem stage when the MMAs retire
-                    if (kb + 1 == kb1) umma_commit(&tmem_full[acc]);     // accumulator complete -> epilogue
+                    __syncwarp();
+                    if (++stage == Cfg::STAGES) { stage = 0; phase ^= 1; }
                 }
-                __syncwarp();
-                if (++stage == Cfg::STAGES) { stage = 0; phase ^= 1; }
-            }
-            if (kb1 <= kb0) {                            // (cannot happen: the launcher never creates an empty split) keep the epilogue's wait finite
-                if (elect_one()) umma_commit(&tmem_full[acc]);
-                __syncwarp();
+                if (kb1 <= kb0) {                        // (cannot happen: the launcher never creates an empty split) keep the epilogue's wait finite
+                    if (elect_one()) umma_commit_pair(&tmem_full[acc]);
+                    __syncwarp();
+                }
             }
         }
     } else if (warp < EPI_WARPS) {
-        // ===================== epilogue warps (TMEM -> registers -> global) =====================
+        // ===================== epilogue warps (TMEM -> registers -> global), this CTA's 128 rows of the pair tile =====================
         const int q = warp & 3;                          // TMEM lane quarter this warp may access (hardware rule: warp id % 4)
         const int half = warp >> 2;                      // column part: the EPI_PARTS warps of a quarter each drain BN / EPI_PARTS columns
         constexpr int PART_COLS = BN / EPI_PARTS;        // columns per warp per tile
@@ -387,27 +411,28 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
         constexpr int SLICE = PART_COLS * 2;             // bytes of one staged bias slice
         const uint32_t out_tile = smem_u32(epi_stage) + warp * 2 * EPI_TILE_BYTES;
         const uint32_t aux_tile = out_tile + EPI_TILE_BYTES;
+        const uint32_t tmem_empty_leader = mapa_shared(smem_u32(tmem_empty), 0);
         const unsigned long long seed = (p.drop_thresh != 0u) ? effective_seed(p.seed, p.seed_dev) : 0ull;
         const bool use_aux = p.aux != nullptr && (p.epilogue == DLE_EPI_BIAS_DROPOUT_RESIDUAL || p.epilogue == DLE_EPI_DGELU ||
                                                   p.epilogue == DLE_EPI_ADD);
-        if (use_aux && (int)blockIdx.x < total_units) {  // operand of the very first chunk
-            const int tile = blockIdx.x / p.splits;
-            const int m_blk = tile / p.n_tiles, n_blk = tile - m_blk * p.n_tiles;
-            aux_prefetch(p, (long long)m_blk * BM + q * 32, n_blk * BN + half * PART_COLS, aux_tile, lane);
+        if (use_aux && pair < total_units) {             // operand of the very first chunk
+            const int tile = pair / p.splits;
+            const int m_pair = tile / p.n_tiles, n_blk = tile - m_pair * p.n_tiles;
+            aux_prefetch(p, (long long)(m_pair * 2 + (int)rank) * BM + q * 32, n_blk * BN + half * PART_COLS, aux_tile, lane);
         }
         int it = 0;
-        for (int unit = blockIdx.x; unit < total_units; unit += gridDim.x, ++it) {
+        for (int unit = pair; unit < total_units; unit += num_pairs, ++it) {
             const int tile = unit / p.splits;
-            const int m_blk = tile / p.n_tiles, n_blk = tile - m_blk * p.n_tiles;
+            const int m_pair = tile / p.n_tiles, n_blk = tile - m_pair * p.n_tiles;
             const int acc = it & 1; const uint32_t acc_phase = (it >> 1) & 1;
             // bias slice of this warp's column half -> shared.  The slice of tile it+1 is fetched into two registers at the top of tile it
             // and stored after its last chunk, so the global latency never sits in front of the accumulator (in the epilogue-bound
             // regime the accumulator is already waiting).  The four warps of a half write the same values into the same slice; slices
-            // rotate over three tiles because a warp can run at most one tile ahead of a sibling (tmem_empty needs all eight arrivals).
+            // rotate over three tiles because a warp can run at most one tile ahead of a sibling (tmem_empty needs all arrivals).
             const uint32_t bias_s = smem_u32(epi_bias) + ((it % 3) * EPI_PARTS + half) * SLICE;
             const uint32_t bias_next = smem_u32(epi_bias) + (((it + 1) % 3) * EPI_PARTS + half) * SLICE;
             uint2 bnext = make_uint2(0u, 0u);
-            const bool has_next = p.bias != nullptr && unit + (int)gridDim.x < total_units;
+            const bool has_next = p.bias != nullptr && unit + num_pairs < total_units;
             if (p.bias != nullptr) {
                 if (it == 0) {
                     uint2 b0 = make_uint2(0u, 0u);
@@ -417,7 +442,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
                     __syncwarp();
                 }
                 if (has_next) {
-                    const int tile2 = (unit + (int)gridDim.x) / p.splits;
+                    const int tile2 = (unit + num_pairs) / p.splits;
                     const int n2 = tile2 - (tile2 / p.n_tiles) * p.n_tiles;
                     const int col = n2 * BN + half * PART_COLS + lane * EPL;
                     if (col < p.N) bnext = bias_load<EPL>(p.bias + col);
@@ -425,7 +450,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
             }
             mbar_wait(&tmem_full[acc], acc_phase);
             tc_fence_after();
-            const long long row_base = (long long)m_blk * BM + q * 32;
+            const long long row_base = (long long)(m_pair * 2 + (int)rank) * BM + q * 32;
             const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + acc * BN;
 #pragma unroll 1
             for (int cl = 0; cl < CH; ++cl) {
@@ -437,10 +462,10 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
                     aux_take(aux_tile, lane, a);             // landed while the previous chunk was computed / stored
                     if (cl + 1 < CH) {
                         aux_prefetch(p, row_base, n_blk * BN + (c + 1) * 32, aux_tile, lane);
-                    } else if (unit + (int)gridDim.x < total_units) {
-                        const int tile2 = (unit + (int)gridDim.x) / p.splits;
+                    } else if (unit + num_pairs < total_units) {
+                        const int tile2 = (unit + num_pairs) / p.splits;
                         const int m2 = tile2 / p.n_tiles, n2 = tile2 - m2 * p.n_tiles;
-                        aux_prefetch(p, (long long)m2 * BM + q * 32, n2 * BN + half * PART_COLS, aux_tile, lane);
+                        aux_prefetch(p, (long long)(m2 * 2 + (int)rank) * BM + q * 32, n2 * BN + half * PART_COLS, aux_tile, lane);
                     }
                 } else {
 #pragma unroll
@@ -451,7 +476,7 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
             }
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) mbar_arrive(&tmem_empty[acc]);    // one arrival per epilogue warp
+            if (lane == 0) mbar_arrive_cluster(tmem_empty_leader + acc * 8);    // one arrival per epilogue warp of the pair
             if (has_next) {
                 bias_stage<EPL>(bias_next, lane, bnext);
                 __syncwarp();
@@ -459,9 +484,10 @@ gemm_bf16_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_a, const __gri
         }
     }
 
+    // No CTA leaves (or frees its TMEM) while its peer can still signal its barriers or write its TMEM.
     tc_fence_before();
-    __syncthreads();
-    if (warp == WARP_ALLOC) { tc_fence_after(); tmem_dealloc(tmem_base, Cfg::TMEM_COLS); }
+    cluster_sync();
+    if (warp == WARP_ALLOC) { tc_fence_after(); tmem_dealloc_pair(tmem_base, Cfg::TMEM_COLS); }
 }
 
 // ----------------------------------------------------------------------------------------------
@@ -513,15 +539,16 @@ static int launch_gemm_ew(const dle_gemm_args* a, cudaStream_t stream) {
     using Cfg = GemmCfg<BN, EW>;
     CUtensorMap ta, tb;
     int rc;
-    // K-major operand: matrix [rows, K] -> box {64 (k), rows_per_tile}; MN-major: matrix [K, rows] -> box {64 (m/n), 64 (k)}
+    // K-major operand: matrix [rows, K] -> box {64 (k), rows per CTA}; MN-major: matrix [K, rows] -> box {64 (m/n), 64 (k)}.
+    // Per CTA of a pair: 128 rows of A, BN / 2 rows of B.
     rc = A_MN ? make_tmap_bf16_2d(&ta, a->A, a->K, a->M, a->lda, 64, BK) : make_tmap_bf16_2d(&ta, a->A, a->M, a->K, a->lda, BK, BM);
     if (rc != DLE_OK) return rc;
-    rc = B_MN ? make_tmap_bf16_2d(&tb, a->B, a->K, a->N, a->ldb, 64, BK) : make_tmap_bf16_2d(&tb, a->B, a->N, a->K, a->ldb, BK, BN);
+    rc = B_MN ? make_tmap_bf16_2d(&tb, a->B, a->K, a->N, a->ldb, 64, BK) : make_tmap_bf16_2d(&tb, a->B, a->N, a->K, a->ldb, BK, BN / 2);
     if (rc != DLE_OK) return rc;
 
     GemmKernelParams p;
     p.M = a->M; p.N = a->N; p.K = a->K;
-    p.m_tiles = (a->M + BM - 1) / BM;
+    p.m_tiles = (a->M + 2 * BM - 1) / (2 * BM);
     p.n_tiles = (a->N + BN - 1) / BN;
     p.kb_total = (a->K + BK - 1) / BK;
     int splits = a->splits > 0 ? a->splits : 1;
@@ -545,25 +572,38 @@ static int launch_gemm_ew(const dle_gemm_args* a, cudaStream_t stream) {
     p.colsum_out = reinterpret_cast<float*>(a->colsum_out);
 
     auto kern = gemm_bf16_tcgen05_kernel<BN, A_MN, B_MN, EW>;
-    static bool attr_set[64] = {};                      // the attribute is per device (and per template instance)
+    cudaLaunchConfig_t cfg = {};
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+    cfg.blockDim = dim3(Cfg::THREADS);
+    cfg.dynamicSmemBytes = Cfg::SMEM_BYTES;
+    cfg.stream = stream;
+    cfg.attrs = attr; cfg.numAttrs = 1;
+    // per device (and per template instance): the shared-memory attribute, and how many pairs can be resident at once -- a persistent
+    // grid larger than that would run its last pairs as a second wave
+    static int pair_slots[64] = {};
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return DLE_ERR_CUDA;
-    if (!attr_set[dev]) {
+    if (pair_slots[dev] == 0) {
         if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES) != cudaSuccess)
             return DLE_ERR_CUDA;
-        attr_set[dev] = true;
+        int clusters = 0;
+        cfg.gridDim = dim3(2 * (num_sms() / 2));
+        if (cudaOccupancyMaxActiveClusters(&clusters, kern, &cfg) != cudaSuccess || clusters <= 0) return DLE_ERR_CUDA;
+        pair_slots[dev] = clusters < num_sms() / 2 ? clusters : num_sms() / 2;
     }
     const int units = p.m_tiles * p.n_tiles * p.splits;
-    const int grid = units < num_sms() ? units : num_sms();
-    kern<<<grid, Cfg::THREADS, Cfg::SMEM_BYTES, stream>>>(ta, tb, p);
+    cfg.gridDim = dim3(2 * (units < pair_slots[dev] ? units : pair_slots[dev]));
+    if (cudaLaunchKernelEx(&cfg, kern, ta, tb, p) != cudaSuccess) return DLE_ERR_CUDA;
     DLE_LAUNCH_CHECK();
     return DLE_OK;
 }
 
 template <int BN, bool A_MN, bool B_MN>
 static int launch_gemm(const dle_gemm_args* a, cudaStream_t stream) {
-    // 16 epilogue warps only where they pay (see GemmCfg): the gelu'(u) epilogue on the 256-wide tile
-    if (BN == 256 && a->epilogue == DLE_EPI_DGELU) return launch_gemm_ew<BN, A_MN, B_MN, (BN == 256 ? 16 : 8)>(a, stream);
+    // 16 epilogue warps only where they pay (see GemmCfg)
+    if ((DLE_GEMM_EW16_EPILOGUES >> a->epilogue) & 1u) return launch_gemm_ew<BN, A_MN, B_MN, 16>(a, stream);
     return launch_gemm_ew<BN, A_MN, B_MN, 8>(a, stream);
 }
 

@@ -133,14 +133,14 @@ def _sm_count():
     return n
 
 
-def _split_k(tiles, sms, max_splits):
-    """Split-K factor for a GEMM with `tiles` output tiles on a persistent grid of `sms` CTAs: the smallest factor whose work units fill
-    whole waves (units / (ceil(units / sms) * sms) >= 0.93), else the best found.  Round 1 used ceil(sms / tiles), which left the
-    QKV weight gradient (96 tiles -> 192 units = 1.3 waves) at 1000 TFLOP/s and the attention-output one (32 -> 160 = 1.08 waves) at 750."""
+def _split_k(tiles, slots, max_splits):
+    """Split-K factor for a GEMM with `tiles` output tiles on a persistent grid of `slots` workers: the smallest factor whose work units fill
+    whole waves (units / (ceil(units / slots) * slots) >= 0.93), else the best found.  Round 1 used ceil(slots / tiles), which left the
+    QKV weight gradient (1.3 waves) at 1000 TFLOP/s and the attention-output one (1.08 waves) at 750."""
     best, best_eff = 1, 0.0
     for s_ in range(1, max(1, max_splits) + 1):
         units = tiles * s_
-        eff = units / (-(-units // sms) * sms)
+        eff = units / (-(-units // slots) * slots)
         if eff >= 0.93:
             return s_
         if eff > best_eff + 1e-9:
@@ -150,16 +150,17 @@ def _split_k(tiles, sms, max_splits):
 
 def wgrad(dy, x, out_dtype):
     """dW[N_out, K_in] = dy[T, N_out]^T @ x[T, K_in]; both operands read MN-major where they lie.
-    Few output tiles => split-K over tokens with fp32 red.global.add; otherwise direct store."""
+    Few output tiles => split-K over tokens with fp32 red.global.add; otherwise direct store.
+    The GEMM kernel runs each 256 x 256 output tile on a pair of SMs, so work is counted in pair tiles over SMs / 2 pair slots."""
     T, n_out = dy.shape
     k_in = x.shape[1]
-    tiles = ((n_out + 127) // 128) * ((k_in + 255) // 256)
-    sms = _sm_count()
-    if tiles >= sms * 3 // 4:
+    tiles = ((n_out + 255) // 256) * ((k_in + 255) // 256)
+    slots = _sm_count() // 2
+    if tiles >= slots * 3 // 4:
         if out_dtype == torch.float32:
             return K.gemm(dy, x, a_layout=L.LAYOUT_MN, b_layout=L.LAYOUT_MN, epilogue=L.EPI_F32)
         return K.gemm(dy, x, a_layout=L.LAYOUT_MN, b_layout=L.LAYOUT_MN, epilogue=L.EPI_BIAS)
-    splits = _split_k(tiles, sms, min(16, (T + 511) // 512))
+    splits = _split_k(tiles, slots, min(16, (T + 511) // 512))
     acc = K.gemm(dy, x, a_layout=L.LAYOUT_MN, b_layout=L.LAYOUT_MN, epilogue=L.EPI_ATOMIC_F32, splits=splits)
     return acc if out_dtype == torch.float32 else K.cast_f32_to_bf16(acc)
 
